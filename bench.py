@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the driver's benchmark contract for the fuzzysearch hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input: ONE bounded-Levenshtein
 search (``find_near_matches(pattern, haystack, max_l_dist=2)``, |pattern| = 20) of a 4 GiB
@@ -453,7 +453,13 @@ def main():
                     help="multi-GPU reduction: inside the library over NVLink peer memory (default; 'nccl' is an "
                          "alias), or through torch.distributed (tools/torch_reduce.py, comparison only)")
     ap.add_argument("--ref-cores", type=int, default=0, help="reference arm: processes to use (0 = all cores)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the matches the last timed step returned to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what --impl ours computed")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -482,12 +488,10 @@ def main():
             return 0
         hay = synth_sample_host(alphabet, seed, pat, sample, m, k, kind)
         times, nm = [], 0
-        for i in range(args.warmup + max(args.steps, 5)):  # >= 5 timed steps: the arm is noisy (fork pool)
+        for i in range(args.warmup + args.steps):
             dt, nm = run_reference_sample(hay, pat, kind, k, cores)
             if i >= args.warmup:
                 times.append(dt)
-            if sum(times) > 240:
-                break
         sec = float(np.median(times))
         val = sample / sec / 1e9
         # the reference as it actually ships is single-threaded: one plain find_near_matches call
@@ -578,24 +582,70 @@ def main():
             return h.search_levenshtein(pat, k, gflag)
         return h.search_hamming(pat, k, gflag)
 
-    def step(h=None):
+    def step(h=None, keep=None):
         # one search of this rank's shard (local consolidation on the device); multi-GPU: the per-shard
         # groups are all-gathered by NCCL inside the library, on the search's stream, and merged
-        # (--reduce torch: the same reduction through torch.distributed, for comparison)
+        # (--reduce torch: the same reduction through torch.distributed, for comparison).
+        # With a list as `keep`, the results are appended to it instead of being closed.
         if kind == "batch":
             results, st = (h or hs).search_levenshtein_batch(batch_pats, batch_ks)
             nfinal = sum(r.count(F.FINAL) for r in results)
+            if keep is not None:
+                keep.extend(results)
+                return st, nfinal
             for r in results:
                 r.close()
             return st, nfinal
         res = one_search(h or hs)
         st = res.stats()
         if world > 1 and not in_library:
-            nfinal = len(gather_and_merge_groups(result=res, as_arrays=True)[0])
+            merged = gather_and_merge_groups(result=res, as_arrays=True)
+            nfinal = len(merged[0])
         else:
+            merged = None
             nfinal = res.count(F.FINAL)
+        if keep is not None:
+            keep.append(res if merged is None else merged)
+            if merged is None:
+                return st, nfinal
         res.close()
         return st, nfinal
+
+    def dump_outputs(kept):
+        """What the caller of the timed path receives, as float64 columns: every final match (start, end,
+        dist), plus the pattern index for the batch; a fixed sample of rows if they exceed 64 MiB."""
+        if kind == "batch":
+            cols = {"pattern": [], "start": [], "end": [], "dist": []}
+            for j, r in enumerate(kept):  # this rank's patterns are rank, rank + world, ...
+                s, e, d = r.arrays(F.FINAL)
+                cols["pattern"].append(np.full(len(s), rank + j * world))
+                cols["start"].append(s)
+                cols["end"].append(e)
+                cols["dist"].append(d)
+                r.close()
+            cols = {name: np.concatenate(c) if c else np.zeros(0) for name, c in cols.items()}
+            if dist is not None:
+                box = [None] * world
+                dist.all_gather_object(box, cols)
+                order = np.argsort(np.concatenate([b["pattern"] for b in box]), kind="stable")
+                cols = {name: np.concatenate([b[name] for b in box])[order] for name in cols}
+        else:
+            r = kept[0]
+            s, e, d = r if isinstance(r, tuple) else r.arrays(F.FINAL)
+            if not isinstance(r, tuple):
+                r.close()
+            cols = {"start": s, "end": e, "dist": d}
+        if rank != 0:
+            return
+        n = len(cols["start"])
+        max_rows = (64 << 20) // (8 * (len(cols) + 1))  # + the "row" column of a sample
+        if n > max_rows:
+            rows = np.sort(np.random.default_rng(0).choice(n, max_rows, replace=False))
+            cols = {name: c[rows] for name, c in cols.items()}
+            cols["row"] = rows
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, c in cols.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), np.asarray(c, dtype=np.float64))
 
     def sync_all():
         if dist is not None:
@@ -610,14 +660,17 @@ def main():
     time.sleep(0.3)
     sync_all()
     filt_ms, launches, nfinal = [], 0, 0
+    kept = [] if args.dump_outputs else None
     hs.timer_start()
     t0 = time.perf_counter()
-    for _ in range(args.steps):
-        st, nfinal = step()
+    for i in range(args.steps):
+        st, nfinal = step(keep=kept if i == args.steps - 1 else None)
         filt_ms.append(st["filter_ms"])
         launches += st["n_launches"]
     dev_ms = hs.timer_stop()
     wall_ms = (time.perf_counter() - t0) * 1e3
+    if kept is not None:
+        dump_outputs(kept)
     sync_all()
     # the timed region of a default run lasts ~20 ms, shorter than one nvidia-smi sampling period: keep
     # the SAME searches running (untimed, same count on every rank) so the clock monitor sees the load

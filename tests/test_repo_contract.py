@@ -6,6 +6,9 @@ import re
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -55,7 +58,8 @@ def test_reference_arm_prints_the_contract_line():
     assert line["value"] > 0 and line["cpu_baseline"]["kind"] == "reference" and line["cpu_baseline"]["cores"] == 2
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["value"] == line["value"]
     assert line["config"]["workload"] == "ascii64m_lev_m20_k2" and line["metric"] == "haystack_GB_per_s_scanned"
-    assert line["steps"] >= 5 and line["cpu_baseline"]["single_core_value"] > 0
+    assert line["steps"] == 1 and len(line["cpu_baseline"]["step_values"]) == 1
+    assert line["cpu_baseline"]["single_core_value"] > 0
 
 
 def test_reference_arm_never_loads_the_product_library(tmp_path):
@@ -83,3 +87,26 @@ def test_graft_entry_exposes_build_and_smoke():
     sys.path.insert(0, ROOT)
     import __graft_entry__ as g
     assert callable(g.build) and callable(g.smoke)
+
+
+@pytest.mark.gpu
+def test_bench_dumps_what_the_last_timed_step_returned(tmp_path, cuda_device):
+    """`--steps K` times exactly K searches and `--dump-outputs DIR` writes the final list of the last one; the
+    inputs are seeded, so two runs write the same arrays."""
+    def run(name, steps):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "ascii64m_lev_m20_k2",
+                              "--steps", str(steps), "--warmup", "0", "--e2e-steps", "0", "--no-cpu-baseline",
+                              "--dump-outputs", str(tmp_path / name)], capture_output=True, text=True, timeout=600)
+        assert out.returncode == 0, out.stderr[-2000:]
+        line = json.loads(out.stdout.strip().splitlines()[-1])
+        assert sorted(os.listdir(tmp_path / name)) == ["dist.npy", "end.npy", "start.npy"]
+        return line, {n: np.load(tmp_path / name / (n + ".npy")) for n in ("start", "end", "dist")}
+
+    line1, one = run("one", 1)
+    line3, three = run("three", 3)
+    assert line1["steps"] == 1 and line3["steps"] == 3
+    assert line1["parity"]["ok"] and line1["matches_per_step"] == line1["parity"]["final"] == len(one["start"]) > 0
+    for n in one:
+        assert one[n].dtype == np.float64 and np.array_equal(one[n], three[n]), n
+    assert np.all(one["start"] < one["end"]) and np.all(np.diff(one["start"]) > 0)
+    assert set(np.unique(one["dist"])) <= {0.0, 1.0, 2.0}
