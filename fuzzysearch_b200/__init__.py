@@ -10,7 +10,8 @@ Every search runs as hand-written CUDA kernels behind the C-ABI of libfuzzb200.s
 """
 __version__ = "0.1.0"
 
-__all__ = ["find_near_matches", "find_near_matches_batch", "find_near_matches_in_file", "has_near_match", "Match", "LevenshteinSearchParams",
+__all__ = ["find_near_matches", "find_near_matches_batch", "find_near_matches_in_file", "find_near_matches_in_sequences",
+           "has_near_match", "has_near_match_in_sequences", "Match", "LevenshteinSearchParams",
            "DeviceSequence", "ExactSearch", "SubstitutionsOnlySearch", "LevenshteinSearch",
            "GenericSearch", "choose_search_class", "search_exact"]
 
@@ -83,6 +84,41 @@ def find_near_matches_batch(subsequences, sequence, max_l_dist):
             out.append([Match(a, b, c, matched=slicer(a, b)) for a, b, c in zip(s.tolist(), e.tolist(), d.tolist())])
             res.close()
     return out
+
+
+def find_near_matches_in_sequences(subsequence, sequences, max_substitutions=None, max_insertions=None,
+                                   max_deletions=None, max_l_dist=None):
+    """One pattern over many sequences (reads, lines, records): -> one list of Match per sequence, equal to
+    ``[find_near_matches(subsequence, s, ...) for s in sequences]`` (``Match.matched`` is a slice of that item).
+
+    The items are packed into one buffer and searched in a single device pass (fzb_search_segments) instead of paying
+    the fixed cost of a search per item.  Items may be bytes, bytearray, memoryview, numpy uint8 arrays or str; items
+    with wide symbols, or list / tuple items, are searched one by one."""
+    sequences = list(sequences)
+    if not sequences:
+        return []
+    search_params = LevenshteinSearchParams(max_substitutions, max_insertions, max_deletions, max_l_dist)
+    choose_search_class(search_params)
+    from .search import search_sequences
+
+    def per_item(s):
+        return find_near_matches(subsequence, s, max_substitutions, max_insertions, max_deletions, max_l_dist)
+    return search_sequences(subsequence, sequences, search_params, per_item)
+
+
+def has_near_match_in_sequences(subsequence, sequences, max_substitutions=None, max_insertions=None,
+                                max_deletions=None, max_l_dist=None):
+    """-> one bool per sequence: True where find_near_matches_in_sequences(...) has a non-empty list (e.g. which reads
+    contain the primer)."""
+    sequences = list(sequences)
+    if not sequences:
+        return []
+    search_params = LevenshteinSearchParams(max_substitutions, max_insertions, max_deletions, max_l_dist)
+    from .search import search_sequences
+
+    def per_item(s):
+        return find_near_matches(subsequence, s, max_substitutions, max_insertions, max_deletions, max_l_dist)
+    return search_sequences(subsequence, sequences, search_params, per_item, counts_only=True)
 
 
 def choose_search_class(search_params):

@@ -17,11 +17,13 @@ FZB_E_CUDA = -2
 FZB_E_UNSUPPORTED = -3
 FZB_E_NGRAM_ZERO = -4
 FZB_MAX_PATTERN = 255
+FZB_SEG_SHORT_BYTES = 4096    # segments up to this length are searched one warp each; longer ones one by one
+FZB_SEG_MAX_COUNT = 1 << 23   # segments per fzb_search_segments call (the segment number's bits in a raw record)
 
 RAW, FINAL = 0, 1
 F_NO_FINAL, F_FORCE_DENSE, F_FORCE_LP, F_FORCE_NGRAMS, F_TINY_LIST, F_GLOBAL, F_FORCE_SAMPLED = 1, 2, 4, 8, 16, 32, 64
 
-ROUTE_NAMES = {7: "batch", 0: "exact", 1: "ngrams/sampled-filter", 2: "ngrams/dense-filter", 3: "lp",
+ROUTE_NAMES = {8: "segments", 7: "batch", 0: "exact", 1: "ngrams/sampled-filter", 2: "ngrams/dense-filter", 3: "lp",
                4: "hamming", 5: "generic-ngrams", 6: "generic-lp"}
 
 
@@ -79,6 +81,8 @@ SYMBOLS = {
     "fzb_search_hamming": (_i32, [_vp, _u8p, _u32, _u32, _u32, _vpp]),
     "fzb_search_generic": (_i32, [_vp, _u8p, _u32, _u32, _u32, _u32, _u32, _u32, _vpp]),
     "fzb_search_exact": (_i32, [_vp, _u8p, _u32, _u32, _vpp]),
+    "fzb_search_segments": (_i32, [_vp, _u8p, _u32, _vp, _u64, _u32, _u32, _u32, _u32, _u32, _vpp]),
+    "fzb_result_segment_counts": (_i32, [_vp, _i32, _vp]),
     "fzb_search_exact_window": (_i32, [_vp, _u8p, _u32, _u64, _u64, _u32, _vpp]),
     "fzb_search_levenshtein_batch": (_i32, [_vp, _u8p, _vp, _vp, _u32, _u32, _vpp, ctypes.POINTER(Stats)]),
     "fzb_find_near_matches": (_i32, [_u8p, _u32, _u8p, _u64, _u32, _u32, _u32, _u32, _i32, _vpp]),
@@ -199,6 +203,13 @@ class Result(object):
         if cnt < 0:
             check(int(cnt))
         return rows[:n]
+
+    def segment_counts(self, which=FINAL):
+        """fzb_search_segments results: the length of each segment's `which` list (uint64 array)."""
+        n = int(self._nseg)
+        out = np.empty(n, dtype=np.uint64)
+        check(lib().fzb_result_segment_counts(self._h, which, ptr(out)))
+        return out
 
     def triples(self, which=FINAL):
         s, e, d = self.arrays(which)
@@ -359,6 +370,20 @@ class Haystack(object):
         results = [Result(ctypes.c_void_p(out[i])) for i in range(len(pats))]
         return results, {"gpu_ms": st.gpu_ms, "filter_ms": st.filter_ms, "bytes_scanned": st.bytes_scanned,
                          "n_candidates": st.n_candidates, "n_launches": st.n_launches, "route": "batch"}
+
+    def search_segments(self, pattern, offsets, max_subs, max_ins, max_dels, max_l, flags=0):
+        """One pattern over the segments [offsets[i], offsets[i+1]) of this sequence, each searched as a whole sequence
+        (normalised limits, as for has_near_match).  -> Result with segment-major lists; .segment_counts(which)."""
+        p, pp, m = self._pat(pattern)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        if offsets.ndim != 1 or offsets.size < 1:
+            raise ValueError("offsets must hold count + 1 entries")
+        r = ctypes.c_void_p()
+        check(lib().fzb_search_segments(self._h, pp, m, ptr(offsets), offsets.size - 1, max_subs, max_ins, max_dels,
+                                        max_l, flags, ctypes.byref(r)))
+        res = Result(r)
+        res._nseg = offsets.size - 1
+        return res
 
     def has_near_match(self, pattern, max_subs, max_ins, max_dels, max_l):
         """True iff the search would return at least one match; stops at the first chunk that holds one."""

@@ -27,6 +27,7 @@
 #include "p2p_kernels.cuh"
 #include "batch_kernels.cuh"
 #include "sym_kernels.cuh"
+#include "seg_kernels.cuh"
 #include <unordered_map>
 #include "debug_kernels.cuh"
 
@@ -191,6 +192,17 @@ struct fzb_haystack {
     unsigned long long *d_lmkept = nullptr; // ... the survivors of the exact per-pattern window test
     uint32_t *d_lmhist = nullptr;
     uint32_t lmlist_cap = 0;
+    // segmented searches (seg_kernels.cuh), allocated on first use
+    uint64_t *d_seg_offsets = nullptr;     // the caller's offsets[count + 1]
+    uint32_t *d_seg_cnt = nullptr;         // per segment: raw record counts, then final counts ([2][count])
+    uint32_t *d_seg_off = nullptr, *d_seg_cur = nullptr;
+    uint32_t *h_seg_cnt = nullptr;         // pinned: host copy of d_seg_cnt
+    uint64_t seg_count_cap = 0;
+    uint64_t *d_seg_keys = nullptr;        // canonical keys grouped by segment
+    uint64_t *h_seg_raw = nullptr, *h_seg_fin = nullptr;  // mapped: sorted raw keys / final keys, segment-major
+    uint64_t seg_rec_cap = 0;
+    uint32_t *h_seg_hdr = nullptr;         // mapped: record count, overflow flag of the last attempt
+    fzb_haystack *seg_ws = nullptr;        // long segments are copied here and searched as whole sequences
 };
 
 struct fzb_result {
@@ -212,6 +224,8 @@ struct fzb_result {
     uint32_t gcount = 0;
     std::vector<RawRec> gfin;
     int raw_order = 0;         // 0 generation (ngram, idx) / 1 canonical / 2 generic n-grams (5 fields)
+    bool segmented = false;    // fzb_search_segments: raw / fin are segment-major, seg_n holds the list lengths
+    std::vector<uint64_t> seg_n[2];  // [FZB_RAW] / [FZB_FINAL]: per-segment list lengths
     void order_raw();
     fzb_stats stats{};
 };
@@ -328,6 +342,7 @@ static int alloc_buffer(fzb_haystack *h) {
 }
 
 static void p2p_free(fzb_haystack *h);
+static void seg_free(fzb_haystack *h);
 static int upload_bytes(fzb_haystack *h, uint64_t dst_off, const uint8_t *host, uint64_t n);
 
 extern "C" void fzb_haystack_destroy(fzb_haystack *h) {
@@ -361,6 +376,7 @@ extern "C" void fzb_haystack_destroy(fzb_haystack *h) {
     if (h->h_recv) cudaFreeHost(h->h_recv);
     if (h->comm) nccl_comm_destroy(h->comm);
     p2p_free(h);
+    seg_free(h);
     if (h->h_counters) cudaFreeHost(h->h_counters);
     if (h->h_fin) cudaFreeHost(h->h_fin);
     if (h->d_fin) cudaFree(h->d_fin);
@@ -2715,6 +2731,318 @@ extern "C" int fzb_find_near_matches(const uint8_t *pattern, uint32_t m, const u
     else
         rc = fzb_search_generic(h, pattern, m, max_subs, max_ins, max_dels, max_l, 0, out);
     return rc;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Segmented search: one pattern over the segments [offsets[i], offsets[i+1]) of one resident buffer, each searched as
+// a whole sequence (seg_kernels.cuh).  Short segments: one pass of five kernels whatever their number; long ones:
+// copied device-to-device into a workspace handle and searched with the single-sequence entry points.
+// ------------------------------------------------------------------------------------------------
+static void seg_free(fzb_haystack *h) {
+    if (h->seg_ws) fzb_haystack_destroy(h->seg_ws);
+    h->seg_ws = nullptr;
+    if (h->d_seg_offsets) cudaFree(h->d_seg_offsets);
+    if (h->d_seg_cnt) cudaFree(h->d_seg_cnt);
+    if (h->d_seg_off) cudaFree(h->d_seg_off);
+    if (h->d_seg_cur) cudaFree(h->d_seg_cur);
+    if (h->h_seg_cnt) cudaFreeHost(h->h_seg_cnt);
+    h->d_seg_offsets = nullptr;
+    h->d_seg_cnt = h->d_seg_off = h->d_seg_cur = h->h_seg_cnt = nullptr;
+    h->seg_count_cap = 0;
+    if (h->d_seg_keys) cudaFree(h->d_seg_keys);
+    if (h->h_seg_raw) cudaFreeHost(h->h_seg_raw);
+    if (h->h_seg_fin) cudaFreeHost(h->h_seg_fin);
+    h->d_seg_keys = h->h_seg_raw = h->h_seg_fin = nullptr;
+    h->seg_rec_cap = 0;
+    if (h->h_seg_hdr) cudaFreeHost(h->h_seg_hdr);
+    h->h_seg_hdr = nullptr;
+}
+
+static int ensure_seg_buffers(fzb_haystack *h, uint64_t count, uint64_t recs) {
+    const unsigned mapped = cudaHostAllocMapped | cudaHostAllocPortable;
+    if (!h->h_seg_hdr) CK(cudaHostAlloc(&h->h_seg_hdr, 4 * sizeof(uint32_t), mapped));
+    if (count > h->seg_count_cap) {
+        if (h->d_seg_offsets) CK(cudaFree(h->d_seg_offsets));
+        if (h->d_seg_cnt) CK(cudaFree(h->d_seg_cnt));
+        if (h->d_seg_off) CK(cudaFree(h->d_seg_off));
+        if (h->d_seg_cur) CK(cudaFree(h->d_seg_cur));
+        if (h->h_seg_cnt) CK(cudaFreeHost(h->h_seg_cnt));
+        h->d_seg_offsets = nullptr;
+        h->d_seg_cnt = h->d_seg_off = h->d_seg_cur = h->h_seg_cnt = nullptr;
+        h->seg_count_cap = 0;
+        const uint64_t cap = std::max<uint64_t>(count, 1u << 12);
+        CK(cudaMalloc(&h->d_seg_offsets, (cap + 1) * sizeof(uint64_t)));
+        CK(cudaMalloc(&h->d_seg_cnt, 2 * cap * sizeof(uint32_t)));
+        CK(cudaMalloc(&h->d_seg_off, (cap + 1) * sizeof(uint32_t)));
+        CK(cudaMalloc(&h->d_seg_cur, cap * sizeof(uint32_t)));
+        CK(cudaHostAlloc(&h->h_seg_cnt, 2 * cap * sizeof(uint32_t), cudaHostAllocPortable));
+        h->seg_count_cap = cap;
+    }
+    if (recs > h->seg_rec_cap) {
+        if (h->d_seg_keys) CK(cudaFree(h->d_seg_keys));
+        if (h->h_seg_raw) CK(cudaFreeHost(h->h_seg_raw));
+        if (h->h_seg_fin) CK(cudaFreeHost(h->h_seg_fin));
+        h->d_seg_keys = h->h_seg_raw = h->h_seg_fin = nullptr;
+        h->seg_rec_cap = 0;
+        CK(cudaMalloc(&h->d_seg_keys, recs * sizeof(uint64_t)));
+        CK(cudaHostAlloc(&h->h_seg_raw, recs * sizeof(uint64_t), mapped));
+        CK(cudaHostAlloc(&h->h_seg_fin, recs * sizeof(uint64_t), mapped));
+        h->seg_rec_cap = recs;
+    }
+    return FZB_OK;
+}
+
+static RawRec seg_decode(uint64_t key) {  // canonical_key (kernels.cuh) -> record
+    RawRec r;
+    r.start = (int64_t)(key >> 18);
+    r.end = r.start + (int64_t)((key >> 8) & 0x3FFu);
+    r.dist = (int32_t)(key & 0xFFu);
+    r.idx = -1;
+    r.ngram = -1;
+    return r;
+}
+
+// choose_search_class (__init__.py:60-83) on normalised limits, as fzb_find_near_matches dispatches
+static int seg_search_whole(fzb_haystack *w, const uint8_t *pattern, uint32_t m, uint32_t max_subs, uint32_t max_ins,
+                            uint32_t max_dels, uint32_t max_l, fzb_result **r) {
+    if (max_l == 0) return fzb_search_exact(w, pattern, m, 0, r);
+    if (max_ins == 0 && max_dels == 0) return fzb_search_hamming(w, pattern, m, std::min(max_l, max_subs), 0, r);
+    if (max_l <= std::min(max_subs, std::min(max_ins, max_dels))) return fzb_search_levenshtein(w, pattern, m, max_l, 0, r);
+    return fzb_search_generic(w, pattern, m, max_subs, max_ins, max_dels, max_l, 0, r);
+}
+
+// A segment longer than kSegMaxBytes: device-to-device into the workspace handle, searched there as a whole sequence
+// (the HBM-speed filters of the single-sequence routes); its lists are appended to res.
+static int seg_search_long(fzb_haystack *h, uint64_t lo, uint64_t n, const uint8_t *pattern, uint32_t m,
+                           uint32_t max_subs, uint32_t max_ins, uint32_t max_dels, uint32_t max_l, fzb_result *res,
+                           uint64_t *n_raw, uint64_t *n_fin) {
+    if (!h->seg_ws || round_up(n, 128) + 128 > h->seg_ws->capacity) {
+        if (h->seg_ws) fzb_haystack_destroy(h->seg_ws);
+        h->seg_ws = nullptr;
+        const uint64_t cap = std::max<uint64_t>(n + n / 8, 1u << 20);
+        int rc = fzb_haystack_alloc(cap, 0, cap, 0, cap, h->device, &h->seg_ws, nullptr);
+        if (rc) return rc;
+    }
+    fzb_haystack *w = h->seg_ws;
+    w->buf_len = w->global_len = w->own_hi = n;
+    w->own_lo = 0;
+    w->padded_len = round_up(n, 128) + 128;
+    w->coll_prob = -1.0;
+    CK(cudaMemsetAsync(w->d + n, 0, w->padded_len - n, w->stream));
+    CK(cudaMemcpyAsync(w->d, h->d + lo, n, cudaMemcpyDeviceToDevice, w->stream));
+    fzb_result *r = nullptr;
+    int rc = seg_search_whole(w, pattern, m, max_subs, max_ins, max_dels, max_l, &r);
+    if (rc) return rc;
+    r->order_raw();
+    std::vector<RawRec> raw = r->raw;
+    sort_canonical(raw);
+    for (RawRec &x : raw) {
+        x.idx = -1;
+        x.ngram = -1;
+    }
+    res->raw.insert(res->raw.end(), raw.begin(), raw.end());
+    res->fin.insert(res->fin.end(), r->fin.begin(), r->fin.end());
+    *n_raw = raw.size();
+    *n_fin = r->fin.size();
+    res->stats.n_launches += r->stats.n_launches;
+    res->stats.n_candidates += r->stats.n_candidates;
+    fzb_result_destroy(r);
+    return FZB_OK;
+}
+
+static int search_segments(fzb_haystack *h, const uint8_t *pattern, uint32_t m, const uint64_t *offsets,
+                           uint64_t count, uint32_t max_subs, uint32_t max_ins, uint32_t max_dels, uint32_t max_l,
+                           uint32_t flags, fzb_result *res) {
+    int rc = check_pattern(h, pattern, m);
+    if (rc) return rc;
+    if (flags & FZB_F_GLOBAL) return fail(FZB_E_INVALID, "a segmented search is per handle (no FZB_F_GLOBAL)");
+    if (h->buf_lo != 0 || h->global_len != h->buf_len || h->own_lo != 0 || h->own_hi != h->buf_len)
+        return fail(FZB_E_INVALID, "a segmented search needs a whole (unsharded) sequence");
+    if (count > FZB_SEG_MAX_COUNT) return fail(FZB_E_UNSUPPORTED, "more than %u segments in one call", FZB_SEG_MAX_COUNT);
+    if (!offsets) return fail(FZB_E_INVALID, "offsets is NULL");
+    if (offsets[count] > h->global_len) return fail(FZB_E_INVALID, "offsets[count] beyond the end of the sequence");
+    uint64_t short_bytes = 0;
+    for (uint64_t i = 0; i < count; i++) {
+        if (offsets[i] > offsets[i + 1]) return fail(FZB_E_INVALID, "offsets must not decrease");
+        if (offsets[i + 1] - offsets[i] <= (uint64_t)kSegMaxBytes) short_bytes += offsets[i + 1] - offsets[i];
+    }
+    res->segmented = true;
+    res->unconsolidated = max_l == 0 || (max_ins == 0 && max_dels == 0);
+    res->raw_ordered = true;  // segment-major, (start, end, dist) within a segment
+    res->raw_order = 1;
+    res->have_fin = true;
+    res->stats.route = 8;
+    res->stats.bytes_scanned = short_bytes;
+    res->seg_n[FZB_RAW].assign(count, 0);
+    res->seg_n[FZB_FINAL].assign(count, 0);
+    if (count == 0) return FZB_OK;
+    // the route depends on m and the limits only (fzb_search_levenshtein / _hamming / _generic / _exact)
+    SegParams sp;
+    memset(&sp, 0, sizeof sp);
+    memcpy(sp.P, pattern, m);
+    sp.m = (int)m;
+    int route;
+    if (max_l == 0) {
+        route = SEG_EXACT;
+    } else if (max_ins == 0 && max_dels == 0) {
+        route = SEG_HAMMING;
+        sp.k = (int)std::min(std::min(max_l, max_subs), m);
+    } else if (max_l <= std::min(max_subs, std::min(max_ins, max_dels))) {
+        const uint32_t k = std::min(max_l, m);  // every k >= m takes the same branch (levenshtein.py:62-65)
+        sp.k = (int)k;
+        route = m / (k + 1) >= 3 ? SEG_LEV_NGRAMS : SEG_LEV_LP;
+    } else {
+        const bool ngrams = m / (max_l + 1) >= 3;
+        uint32_t l = max_l;  // the LP clamp and the limits of search_generic
+        if (!ngrams) l = (uint32_t)std::min<uint64_t>(l, (uint64_t)m + std::min(max_ins, l));
+        if (l > 63) return fail(FZB_E_UNSUPPORTED, "max_l_dist > 63 is not supported by the generic search");
+        sp.k = (int)l;
+        sp.max_subs = (int)std::min(max_subs, l);
+        sp.max_ins = (int)std::min(max_ins, l);
+        sp.max_dels = (int)std::min(max_dels, l);
+        route = ngrams ? SEG_GEN_NGRAMS : SEG_GEN_LP;
+    }
+    if (route == SEG_LEV_NGRAMS || route == SEG_GEN_NGRAMS) {
+        sp.L = (int)m / (sp.k + 1);
+        sp.n_ngrams = (int)m / sp.L;
+    }
+    const int vm = route == SEG_LEV_NGRAMS ? verify_mode((int)m, sp.L) : 0;
+    const bool lp = route == SEG_LEV_LP || route == SEG_GEN_LP || route == SEG_GEN_NGRAMS;
+    const int consolidate = res->unconsolidated ? 0 : 1;
+    CK(cudaSetDevice(h->device));
+    detach_pending(h);  // the records of this search overwrite the output buffer an earlier result may point at
+    h->counters_clean = false;
+    rc = ensure_seg_buffers(h, count, h->out_cap);
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(h->d_seg_offsets, offsets, (count + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, h->stream));
+    sp.H = h->d;
+    sp.offsets = h->d_seg_offsets;
+    sp.count = (uint32_t)count;
+    sp.counters = h->d_counters;
+    const int grid = (int)std::min<uint64_t>((uint64_t)h->sm_count * 8, (count + kSegWarps - 1) / kSegWarps);
+    const int post_grid = (int)std::min<uint64_t>((uint64_t)h->sm_count * 4, (count + 32 * kSegWarps - 1) / (32 * kSegWarps));
+    int cap = lp ? 256 : 0;
+    uint32_t n = 0;
+    for (int attempt = 0;; attempt++) {
+        if (attempt == 16) return fail(FZB_E_CUDA, "output buffer kept overflowing");
+        if (lp) {
+            rc = ensure_scratch(h, (uint64_t)grid * kSegThreads * 2 * (uint64_t)cap);
+            if (rc) return rc;
+        }
+        rc = ensure_seg_buffers(h, count, h->out_cap);
+        if (rc) return rc;
+        cudaStream_t st = h->stream;
+        CK(cudaMemsetAsync(h->d_counters, 0, CNT_COUNT * sizeof(uint32_t), st));
+        CK(cudaMemsetAsync(h->d_seg_cnt, 0, count * sizeof(uint32_t), st));
+        CK(cudaEventRecord(h->ev[0], st));
+        uint32_t *scr = h->d_scratch;
+        switch (route) {
+        case SEG_EXACT: k_seg_search<SEG_EXACT, 0><<<grid, kSegThreads, 0, st>>>(sp, scr, cap, h->d_out, h->out_cap); break;
+        case SEG_HAMMING: k_seg_search<SEG_HAMMING, 0><<<grid, kSegThreads, 0, st>>>(sp, scr, cap, h->d_out, h->out_cap); break;
+        case SEG_LEV_LP: k_seg_search<SEG_LEV_LP, 0><<<grid, kSegThreads, 0, st>>>(sp, scr, cap, h->d_out, h->out_cap); break;
+        case SEG_GEN_LP: k_seg_search<SEG_GEN_LP, 0><<<grid, kSegThreads, 0, st>>>(sp, scr, cap, h->d_out, h->out_cap); break;
+        case SEG_GEN_NGRAMS: k_seg_search<SEG_GEN_NGRAMS, 0><<<grid, kSegThreads, 0, st>>>(sp, scr, cap, h->d_out, h->out_cap); break;
+        default:
+            if (vm == 0)
+                k_seg_search<SEG_LEV_NGRAMS, 0><<<grid, kSegThreads, 0, st>>>(sp, scr, cap, h->d_out, h->out_cap);
+            else if (vm == 1)
+                k_seg_search<SEG_LEV_NGRAMS, 1><<<grid, kSegThreads, 0, st>>>(sp, scr, cap, h->d_out, h->out_cap);
+            else
+                k_seg_search<SEG_LEV_NGRAMS, 2><<<grid, kSegThreads, 0, st>>>(sp, scr, cap, h->d_out, h->out_cap);
+        }
+        k_seg_hist<<<h->sm_count * 4, kSegSortThreads, 0, st>>>(h->d_out, h->out_cap, h->d_counters, h->d_seg_cnt);
+        k_seg_scan<<<1, kPostThreads, 0, st>>>(h->d_seg_cnt, (uint32_t)count, h->d_counters, h->out_cap, h->d_seg_off,
+                                               h->d_seg_cur, h->h_seg_hdr);
+        k_seg_scatter<<<h->sm_count * 4, kSegSortThreads, 0, st>>>(h->d_out, h->out_cap, h->d_counters, h->d_seg_cur,
+                                                                   h->d_seg_keys);
+        k_seg_post<<<post_grid, kSegThreads, 0, st>>>(h->d_seg_cnt, h->d_seg_off, (uint32_t)count, h->d_seg_keys,
+                                                      h->d_counters, h->out_cap, consolidate, h->d_seg_cnt + count,
+                                                      h->h_seg_raw, h->h_seg_fin);
+        CK(cudaGetLastError());
+        res->stats.n_launches += 5;
+        CK(cudaMemcpyAsync(h->h_seg_cnt, h->d_seg_cnt, 2 * count * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        CK(cudaEventRecord(h->ev[2], st));
+        CK(cudaStreamSynchronize(st));  // the only synchronisation of an attempt
+        n = h->h_seg_hdr[0];
+        if (n > h->out_cap) {
+            rc = ensure_out_cap(h, n);
+            if (rc) return rc;
+            continue;
+        }
+        if (h->h_seg_hdr[1]) {  // an LP candidate list overflowed: more room per lane
+            if (cap >= (1 << 16)) return fail(FZB_E_UNSUPPORTED, "candidate explosion: more than 65536 live candidates for one start");
+            cap *= 8;
+            continue;
+        }
+        break;
+    }
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, h->ev[0], h->ev[2]);
+    res->stats.gpu_ms = res->stats.filter_ms = ms;
+    res->stats.n_candidates = count;
+    const uint32_t *raw_n = h->h_seg_cnt, *fin_n = h->h_seg_cnt + count;
+    res->raw.reserve(n);
+    uint64_t off = 0;
+    std::vector<RawRec> one;
+    for (uint64_t s = 0; s < count; s++) {
+        const uint64_t len = offsets[s + 1] - offsets[s];
+        if (len > (uint64_t)kSegMaxBytes) {
+            rc = seg_search_long(h, offsets[s], len, pattern, m, max_subs, max_ins, max_dels, max_l, res,
+                                 &res->seg_n[FZB_RAW][s], &res->seg_n[FZB_FINAL][s]);
+            if (rc) return rc;
+            continue;
+        }
+        const uint32_t nr = raw_n[s];
+        const size_t r0 = res->raw.size();
+        for (uint32_t i = 0; i < nr; i++) res->raw.push_back(seg_decode(h->h_seg_raw[off + i]));
+        if (fin_n[s] == kSegNoFinal) {  // too many records for a warp: sorted and consolidated here
+            std::sort(res->raw.begin() + r0, res->raw.end(), [](const RawRec &a, const RawRec &b) {
+                if (a.start != b.start) return a.start < b.start;
+                if (a.end != b.end) return a.end < b.end;
+                return a.dist < b.dist;
+            });
+        }
+        if (!consolidate) {
+            res->fin.insert(res->fin.end(), res->raw.begin() + r0, res->raw.end());
+            res->seg_n[FZB_FINAL][s] = nr;
+        } else if (fin_n[s] == kSegNoFinal) {
+            consolidate_recs(std::vector<RawRec>(res->raw.begin() + r0, res->raw.end()), one);
+            res->fin.insert(res->fin.end(), one.begin(), one.end());
+            res->seg_n[FZB_FINAL][s] = one.size();
+        } else {
+            for (uint32_t g = 0; g < fin_n[s]; g++) res->fin.push_back(seg_decode(h->h_seg_fin[off + g]));
+            res->seg_n[FZB_FINAL][s] = fin_n[s];
+        }
+        res->seg_n[FZB_RAW][s] = nr;
+        off += nr;
+    }
+    res->raw_n = (uint32_t)res->raw.size();
+    return FZB_OK;
+}
+
+extern "C" int fzb_search_segments(fzb_haystack *h, const uint8_t *pattern, uint32_t m, const uint64_t *offsets,
+                                   uint64_t count, uint32_t max_subs, uint32_t max_ins, uint32_t max_dels,
+                                   uint32_t max_l_dist, uint32_t flags, fzb_result **out) {
+    HandleLock handle_lock(h);
+    fzb_result *res;
+    int rc = make_result(out, &res);
+    if (rc) return rc;
+    rc = search_segments(h, pattern, m, offsets, count, max_subs, max_ins, max_dels, max_l_dist, flags, res);
+    if (rc) {
+        fzb_result_destroy(res);
+        return rc;
+    }
+    *out = res;
+    return FZB_OK;
+}
+
+extern "C" int fzb_result_segment_counts(const fzb_result *r, int which, uint64_t *counts) {
+    if (!r) return fail(FZB_E_INVALID, "result is NULL");
+    if (!r->segmented) return fail(FZB_E_INVALID, "not the result of a segmented search");
+    const std::vector<uint64_t> &v = r->seg_n[which == FZB_RAW ? FZB_RAW : FZB_FINAL];
+    if (!counts && !v.empty()) return fail(FZB_E_INVALID, "counts is NULL");
+    std::copy(v.begin(), v.end(), counts);
+    return FZB_OK;
 }
 
 // ------------------------------------------------------------------------------------------------

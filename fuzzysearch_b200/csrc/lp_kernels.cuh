@@ -429,7 +429,9 @@ __device__ __forceinline__ bool g_push(uint32_t *list, int &n, int cap, uint32_t
 // Candidates born at `start`, over the sequence that ends (exclusive) at `seq_end` (both global).
 // anchor_idx / anchor_ngram tag the emitted records (n-gram hit that opened the window, or start).
 // H[g] must be the haystack byte at global position g (global memory, or the staged window).
-__device__ bool sim_generic(const ScanParams &p, const uint8_t *sP, const uint8_t *H, int64_t start,
+// PT: ScanParams, or the per-segment context of seg_kernels.cuh (anything with m, k, max_subs, max_ins, max_dels).
+template <class PT>
+__device__ bool sim_generic(const PT &p, const uint8_t *sP, const uint8_t *H, int64_t start,
                             int64_t seq_end, uint32_t *A, uint32_t *B, int cap, int64_t anchor_idx,
                             int anchor_ngram, RawRec *out, uint32_t ocap, uint32_t *counters) {
     const int m = p.m, max_l = p.k, max_subs = p.max_subs, max_ins = p.max_ins, max_dels = p.max_dels;

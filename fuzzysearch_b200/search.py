@@ -29,7 +29,7 @@ def _text(seq):
 
 
 __all__ = ["DeviceSequence", "ExactSearch", "SubstitutionsOnlySearch", "LevenshteinSearch",
-           "GenericSearch", "RawMatches", "search_exact"]
+           "GenericSearch", "RawMatches", "search_exact", "search_sequences"]
 
 
 class DeviceSequence(object):
@@ -427,3 +427,86 @@ class GenericSearch(FuzzySearchBase):
     @classmethod
     def extra_items_for_chunked_search(cls, subsequence, search_params):
         return max(x for x in [search_params.max_l_dist, search_params.max_insertions] if x is not None)
+
+
+def _pack_sequences(subsequence, sequences):
+    """-> (pattern u8, packed bytes, offsets uint64[n + 1], slicers) when the pattern and every item have single-byte
+    symbols of one kind, else None (wide symbols or list / tuple items: no byte alphabet shared by all the items).
+    Raises the TypeError find_near_matches raises for an item of the other kind."""
+    pattern = _text(subsequence)
+    kind = _kind(pattern)
+    if kind == "items" or any(isinstance(s, DeviceSequence) for s in sequences):
+        return None
+    pat = _narrow(pattern, kind)
+    parts, slicers = [], []
+    for original in sequences:
+        seq = _text(original)
+        if _kind(seq) != kind:
+            raise TypeError("subsequence and sequence must both be str or both be byte-like")
+        if kind == "str" or isinstance(seq, (bytes, bytearray)):
+            part = seq.encode("latin-1") if kind == "str" and pat is not None else seq
+            parts.append(part)
+            slicers.append(original)
+        else:
+            host = _native.as_u8(seq)
+            parts.append(host)
+            slicers.append(memoryview(host))
+    if pat is None:
+        return None
+    lengths = np.fromiter((len(x) for x in parts), dtype=np.uint64, count=len(parts))
+    blob = b"".join(parts)
+    offsets = np.zeros(len(parts) + 1, dtype=np.uint64)
+    np.cumsum(lengths, out=offsets[1:])
+    return pat, blob, offsets, slicers
+
+
+def search_sequences(subsequence, sequences, search_params, per_item, counts_only=False):
+    """find_near_matches of one pattern in each of `sequences` through fzb_search_segments: one upload of all the items
+    packed back to back and one native call per FZB_SEG_MAX_COUNT items (the segment number's bits in a raw record).
+    -> one list of Match per item (counts_only: one bool per item, true where that list is non-empty).
+
+    `per_item(sequence)` is the fallback when no byte alphabet is shared by all the items (wide symbols, list / tuple
+    items, resident DeviceSequence items): the items then go one by one, as find_near_matches_batch does."""
+    subs, ins, dels, l = search_params.unpacked
+    if len(subsequence) == 0:
+        raise ValueError("subsequence must not be empty" if l == 0 else "Given subsequence is empty!")
+    try:
+        packed = _pack_sequences(subsequence, sequences)
+    except UnicodeEncodeError:  # a str item outside latin-1
+        packed = None
+    if packed is None:
+        return [bool(per_item(s)) if counts_only else per_item(s) for s in sequences]
+    pat, blob, offsets, slicers = packed
+    big = 1 << 29
+    subs, ins, dels = (big if subs is None else min(subs, big)), (big if ins is None else min(ins, big)), \
+        (big if dels is None else min(dels, big))
+    n_items = len(slicers)
+    out = []
+    with _WORKSPACE_LOCK:
+        hay = _workspace(len(blob))
+        hay.upload(np.frombuffer(blob, dtype=np.uint8))
+        for lo in range(0, n_items, _native.FZB_SEG_MAX_COUNT):
+            hi = min(n_items, lo + _native.FZB_SEG_MAX_COUNT)
+            res = hay.search_segments(pat, offsets[lo:hi + 1], subs, ins, dels, l)
+            try:
+                counts = res.segment_counts(_native.FINAL).tolist()
+                if counts_only:
+                    out.extend(c > 0 for c in counts)
+                    continue
+                starts, ends, dists = (a.tolist() for a in res.arrays(_native.FINAL))
+            finally:
+                res.close()
+            pos = 0
+            for i, c in enumerate(counts):
+                if not c:
+                    out.append([])
+                    continue
+                src = slicers[lo + i]
+                if isinstance(src, memoryview):
+                    out.append([Match(a, b, d, matched=bytes(src[a:b]))
+                                for a, b, d in zip(starts[pos:pos + c], ends[pos:pos + c], dists[pos:pos + c])])
+                else:
+                    out.append([Match(a, b, d, matched=src[a:b])
+                                for a, b, d in zip(starts[pos:pos + c], ends[pos:pos + c], dists[pos:pos + c])])
+                pos += c
+    return out

@@ -213,6 +213,31 @@ int fzb_search_levenshtein_batch(fzb_haystack *h, const uint8_t *patterns, const
                                  const uint32_t *max_l_dist, uint32_t count, uint32_t flags,
                                  fzb_result **out, struct fzb_stats_s *total);
 
+/*
+ * One pattern over MANY sequences in one device pass: the segments [offsets[i], offsets[i+1]) (i < count) of the
+ * whole-sequence handle `h` (offsets non-decreasing, offsets[count] <= its length), each searched as if it were the
+ * whole sequence -- window clipping at 0 and at the segment's own length, positions in the results segment-local.
+ * The limits are the already normalised ones of LevenshteinSearchParams (as for fzb_find_near_matches), and the route
+ * follows choose_search_class and the rules of the single-sequence entry points: exact (max_l_dist == 0), Hamming,
+ * Levenshtein n-grams / LP, generic n-grams / LP -- chosen from m and the limits only, never from a segment's length.
+ * Segments of up to FZB_SEG_SHORT_BYTES are searched by one warp each (five kernel launches per call, whatever
+ * `count`); a longer segment is copied device-to-device into a workspace and searched with the single-sequence entry
+ * points (their launches add to stats.n_launches).  stats.route = 8 (segments).
+ * Lists (fzb_result_copy) are segment-major; fzb_result_segment_counts gives each segment's share:
+ *   FZB_FINAL  each segment's consolidate_matches result in (start, end, dist) order (exact / Hamming: its raw list);
+ *   FZB_RAW    each segment's raw multiset in (start, end, dist) order -- NOT the reference's generation order;
+ *              no anchors.
+ * FZB_F_GLOBAL and sharded handles are refused (FZB_E_INVALID); more than FZB_SEG_MAX_COUNT segments per call
+ * (the segment number travels in 23 bits of each raw record) is FZB_E_UNSUPPORTED.
+ */
+#define FZB_SEG_SHORT_BYTES 4096
+#define FZB_SEG_MAX_COUNT (1u << 23)
+int fzb_search_segments(fzb_haystack *h, const uint8_t *pattern, uint32_t m, const uint64_t *offsets, uint64_t count,
+                        uint32_t max_subs, uint32_t max_ins, uint32_t max_dels, uint32_t max_l_dist, uint32_t flags,
+                        fzb_result **out);
+/* counts[0 .. count) = the length of each segment's `which` list (results of fzb_search_segments only). */
+int fzb_result_segment_counts(const fzb_result *r, int which, uint64_t *counts);
+
 /* ExactSearch.search (search_exact.py:80-85): all (overlapping) occurrences. FINAL == RAW. */
 int fzb_search_exact(fzb_haystack *h, const uint8_t *pattern, uint32_t m, uint32_t flags,
                      fzb_result **out);
@@ -267,7 +292,7 @@ typedef struct fzb_stats_s {
     uint64_t n_candidates;  /* granules / windows handed to the verify stage */
     uint32_t n_launches;    /* kernels launched */
     uint32_t route;         /* 0 exact, 1 n-grams (sampled filter), 2 n-grams (dense filter), 3 LP,
-                               4 hamming, 5 generic n-grams, 6 generic LP */
+                               4 hamming, 5 generic n-grams, 6 generic LP, 8 segments (fzb_search_segments) */
 } fzb_stats;
 int fzb_result_stats(const fzb_result *r, fzb_stats *out);
 void fzb_result_destroy(fzb_result *r);
